@@ -2,7 +2,7 @@
 """bench.py — LM iterations/sec of the calibration solve (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload target] [--scaling weak|strong]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
 A "step" is one trust-region (LM) iteration over the whole synthetic problem: solve the damped
 arrow system, update the state, evaluate residuals + Jacobians at the trial point (reprojection
@@ -28,6 +28,11 @@ line is printed by rank 0.  The default workload is the one `north_star` quotes 
                workload itself sharded over N GPUs, `value` = joint iterations/s.  Before timing,
                a small joint problem is solved sharded and on rank 0 alone: `mg_parity`.
 * --impl reference — the oracle port on all host threads on the SAME (joint) problem.
+* --dump-outputs DIR — after the timed runs, what the last of them returns to a caller: the solved state (one
+               DIR/<name>.npy per array of Calibrator.state(), frames of all ranks joined) and its initial / final
+               cost, all float64.  The inputs are seeded, so two builds can be compared output for output.
+
+Nothing is written into the source tree (it may be read-only): no bytecode caches, outputs only under DIR.
 """
 from __future__ import annotations
 
@@ -43,6 +48,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 from vicalib_b200 import synth  # noqa: E402
 
@@ -323,6 +329,24 @@ def mg_parity_check(dist, Calibrator, new_cal, rank, world, local, inertial, mod
     return res[0]
 
 
+def dump_outputs(out_dir, st, summary, pj, dist, rank, world):
+    """DIR/<name>.npy for every array the timed solve returns; with frame shards rank 0 writes the joint trajectory
+    (each rank's own frames, ghost frames dropped)"""
+    out = {k: np.asarray(v, dtype=np.float64) for k, v in st.items()}
+    out["initial_cost"] = np.float64(summary["initial_cost"])
+    out["final_cost"] = np.float64(summary["final_cost"])
+    if world > 1:
+        f0, f1 = synth.shard_frames(pj.n_frames, rank, world)
+        parts = [None] * world
+        dist.all_gather_object(parts, (out["T_wp"][: f1 - f0], out["v_w"][: f1 - f0]))
+        out["T_wp"] = np.concatenate([t for t, _ in parts])
+        out["v_w"] = np.concatenate([v for _, v in parts])
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for k, v in out.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def run_ours(args):
     from vicalib_b200.capi import Calibrator
 
@@ -367,13 +391,16 @@ def run_ours(args):
     sampler = ClockSampler(local)
     sampler.start()
     time.sleep(0.25)
-    s = g.iterate(steps)
+    s = s_last = g.iterate(steps)
     reps = [s["device_seconds"]]
     t_end = time.time() + 1.0  # extra timed repeats keep the clock sampler busy long enough to see the loaded clocks
     while time.time() < t_end and len(reps) < 50:
         g.load(p)
-        reps.append(g.iterate(steps)["device_seconds"])
+        s_last = g.iterate(steps)
+        reps.append(s_last["device_seconds"])
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, g.state(), s_last, pj, dist, rank, world)
     dev_s = float(np.median(reps))
     launches = s["kernel_launches"]
     persistent = launches <= 3 * steps + 8
@@ -549,7 +576,9 @@ def run_reference(args):
     # W warm-up iterations and K timed ones; on the N-block joint problems the sample is bounded to keep the arm
     # within minutes (an iteration of the 8-block target problem takes seconds on the host)
     k = args.steps if world == 1 else max(2, min(args.steps, 16 // world))
-    rate, t_all, _, _ = oracle_rate(p, threads, k, warm=max(1, min(args.warmup, 2)))
+    rate, t_all, o, s = oracle_rate(p, threads, k, warm=max(1, min(args.warmup, 2)))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, o.state(), s, p, None, 0, 1)
     v = rate * mult
     cb = {"value": v, "unit": UNIT, "cores": threads, "kind": "port",
           "sample": f"{k} LM iterations of the {'joint ' if world > 1 else ''}problem ({p.n_obs} observations, "
@@ -580,7 +609,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-flush", action="store_true")
     ap.add_argument("--parity-iters", type=int, default=10, help="iterations of the GPU-vs-oracle parity run (0: skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed run returns as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly one JSON line: library chatter (e.g. NCCL's version banner) goes to stderr
     global _RESULT_FD
     sys.stdout.flush()
